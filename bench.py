@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            (N>1: launched by torch.distributed.run, one rank per GPU)
     python bench.py --impl reference ...                      (the reference's CPU path = the oracle port, host cores)
     python bench.py --workload frame-ring|frame-uniform|stress
+    python bench.py ... --dump-outputs DIR                    (also write the detections of the last timed step as DIR/<name>.npy)
 
 Workloads (BASELINE.json `configs`; SURVEY.md 8(d) inputs, generators in se-ssd_b200/sessd_data/synth.py):
   frame-ring     configs[1]: car-only inference, batch 1 per launch, full path voxelise -> sparse 3-D encoder -> BEV neck/head ->
@@ -28,6 +29,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the source tree, which may be read-only
 for _p in (ROOT, os.path.join(ROOT, "se-ssd_b200"), os.path.join(ROOT, "scripts")):
     if _p not in sys.path:
         sys.path.insert(0, _p)
@@ -51,7 +53,12 @@ def parse():
     ap.add_argument("--cg-deep", type=int, default=None, help="sparse conv pipeline: 1 deep / one CTA per SM, 0 two CTAs per SM (default: the engine's choice)")
     ap.add_argument("--quick", action="store_true", help="skip the e2e / roofline / cpu_baseline / extra legs (tuning runs)")
     ap.add_argument("--no-extra", action="store_true", help="skip the extra.uniform20k / extra.stress sub-records")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the detections computed in the last one as DIR/<name>.npy (see dump_outputs)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
 
 
 # ------------------------------------------------------------------------------------------------------------------ workloads
@@ -83,6 +90,22 @@ def bench_weights(wl):
     from sessd_data import weights
     layers, ssfa, head = weights.bench_detector_state(WORKLOADS[wl]["cloud"], 0)
     return layers, ssfa, head, weights.kitti_car_anchors()
+
+
+def dump_outputs(path, frames):
+    """--dump-outputs: `frames` are dicts of FrameEngine.results() (box3d_lidar, scores, label_preds, anchor_index) plus `cloud`, the
+    index of the frame's input in the seeded cloud pool.  Writes path/<name>.npy: cloud and num_detections per frame, the detections
+    of all frames concatenated in frame order; box3d_lidar / scores in float32, integers in float64 (exact)."""
+    out = {"cloud": np.float64([d["cloud"] for d in frames]),
+           "num_detections": np.float64([len(d["scores"]) for d in frames]),
+           "box3d_lidar": np.concatenate([np.asarray(d["box3d_lidar"], np.float32).reshape(-1, 7) for d in frames]),
+           "scores": np.concatenate([np.asarray(d["scores"], np.float32) for d in frames]),
+           "label_preds": np.concatenate([np.asarray(d["label_preds"], np.float64) for d in frames]),
+           "anchor_index": np.concatenate([np.asarray(d["anchor_index"], np.float64) for d in frames])}
+    assert sum(a.nbytes for a in out.values()) <= 64 << 20
+    os.makedirs(path, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------------------------
@@ -150,7 +173,7 @@ def cpu_frames(wl, clouds, layers, ssfa, head, anchors, n, warm=1):
 
 
 def run_reference(args):
-    """--impl reference: the CPU path timed on the box's host cores; each step = ONE frame (bounded sample).  Imports only oracle/ and
+    """--impl reference: the CPU path timed on the box's host cores; each step = ONE frame (warm-up bounded in time).  Imports only oracle/ and
     the library-free sessd_data generators: libsessd_b200.so is NOT loaded in this arm."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
@@ -169,22 +192,24 @@ def run_reference(args):
     warm = max(0, min(args.warmup - 1, int(0.25 * budget_s / max(t_first, 1e-3))))
     for i in range(warm):
         oframe.frame_detections(clouds[(i + 1) % len(clouds)], lnp, ssfa, head, anchors, max_voxels=mv)
-    spent = time.perf_counter() - t0
-    per_frame = spent / (1 + warm)
-    steps = max(1, min(args.steps, int((budget_s - spent) / max(per_frame, 1e-3))))
+    steps = args.steps
     stage = {}
     t0 = time.perf_counter()
     for i in range(steps):
-        oframe.frame_detections(clouds[i % len(clouds)], lnp, ssfa, head, anchors, max_voxels=mv, timings=stage)
+        last = oframe.frame_detections(clouds[i % len(clouds)], lnp, ssfa, head, anchors, max_voxels=mv, timings=stage)
     dt = time.perf_counter() - t0
     fps = steps / dt
+    if args.dump_outputs:
+        boxes, scores, labels, aux = last
+        dump_outputs(args.dump_outputs, [dict(box3d_lidar=boxes, scores=scores, label_preds=labels, anchor_index=aux["final_anchor"],
+                                              cloud=(steps - 1) % len(clouds))])
     line = {"impl": "reference", "metric": "frames_per_sec", "value": fps, "unit": "frames/s", "n_gpus": args.gpus, "steps": args.steps,
             "warmup": args.warmup, "timed_steps": steps, "timed_warmup": 1 + warm, "ms_per_step": 1000.0 * dt / steps, "higher_is_better": True,
             "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic", "config": workload_config(wl),
             "run": {"frames_per_step": 1, "note": "CPU oracle port of the reference path, rank 0 only"},
             "cpu_baseline": {"value": fps, "unit": "frames/s", "cores": min(CPU_THREADS, os.cpu_count() or 1),
                              "host_threads_available": os.cpu_count() or 1, "kind": "port",
-                             "sample": "%d frames timed (1 frame per step, capped to a ~3 min run), %d warm-up; per-frame stage seconds %s; the sparse "
+                             "sample": "%d frames timed (1 frame per step), %d warm-up; per-frame stage seconds %s; the sparse "
                                        "encoder has no CPU implementation in the reference (spconv is GPU/third-party): numpy restatement" % (
                                            steps, 1 + warm, {k: round(v / steps, 3) for k, v in stage.items()})},
             "e2e": {"value": fps, "unit": "frames/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
@@ -273,6 +298,17 @@ class Rig:
                     e.graph_dev.replay()
         return fn
 
+    def last_step_outputs(self, s, F):
+        """What the engines still hold after step s of step_device(F): the detections of every engine's last launch in that step, in
+        launch order (a fixed subset of the step's frames), unpacked by FrameEngine.results()."""
+        S, frames = len(self.engines), []
+        for i in range(max(0, F // self.B - S), F // self.B):
+            e = self.engines[i % S]
+            e.h_result.copy_(e.d_result)
+            e.h_meta.copy_(e.d_meta)
+            frames += [dict(d, cloud=j) for j, d in zip(self.batch_ids(s, i, F), e.results())]
+        return frames
+
     def prime_offsets(self):
         """frame offsets of the device-resident loop (all pool clouds have the same point count in these workloads)"""
         for e in self.engines:
@@ -333,6 +369,8 @@ def run_ours(args):
     ms_value = rig.timed(fn, args.steps)
     clocks = sampler.stop()
     value = world * F * args.steps / (ms_value / 1000.0)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, rig.last_step_outputs(args.steps - 1, F))
 
     if args.quick:
         if rank == 0:

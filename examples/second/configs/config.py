@@ -1,7 +1,7 @@
 """SE-SSD car detector on KITTI -- hot-path configuration for the B200 build.
 
 Same variable names, registry type strings and hyper-parameters as the reference's examples/second/configs/config.py (which also
-loads unchanged through this repo's ``det3d`` package: tests/test_compat.py does that when the reference tree is present);
+loads unchanged through this repo's ``det3d`` package: tests/test_compat.py checks that both build the same detector);
 dataset paths, augmentation, optimiser and runtime sections of the reference are out of the hot path and omitted here."""
 import itertools
 import logging

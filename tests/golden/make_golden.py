@@ -12,9 +12,14 @@ so only outputs -- or their hashes when large -- are stored):
   decode_case.npz      reference box_torch_ops.second_box_decode
   ssfa_head_case.npz   reference SSFA + Head modules (rpn_v1.py, mg_head_sessd.py) with seeded state dicts
   vfe_case.npz         reference VoxelFeatureExtractorV3
+  iou_self_case.npz    reference iou3d_cpu.cpp: BEV IoU of 150 seeded boxes against themselves
+  reference_config_detector.json
+                       the detector this repo's det3d builds from the reference's unchanged examples/second config:
+                       state-dict layout, parameter count, test_cfg and assigner output stride
 """
 import hashlib
 import importlib.util
+import json
 import os
 import sys
 import types
@@ -89,6 +94,33 @@ def gen_iou():
     assert (ocpu.boxes_iou_bev(a5, c5) == iou.numpy()).all()
     np.savez_compressed(os.path.join(HERE, "iou_cases.npz"), overlap=ov.numpy(), iou=iou.numpy())
     print("iou", ov.shape, float(ov.max()), int((ov > 0).sum()))
+
+
+def gen_iou_self():
+    ref = obuild.load_ref() or (obuild.build_ref() and obuild.load_ref())
+    b, _ = synth.random_boxes(99, 150, spread=0.2)
+    a5 = ocpu.boxes3d_to_bev(b)
+    iou = torch.zeros(150, 150)
+    ref.boxes_iou_bev_cpu(torch.from_numpy(a5), torch.from_numpy(a5), iou)
+    assert (ocpu.boxes_iou_bev(a5, a5) == iou.numpy()).all()
+    np.savez_compressed(os.path.join(HERE, "iou_self_case.npz"), iou=iou.numpy())
+    print("iou self", iou.shape, int((iou > 0).sum()))
+
+
+# --------------------------------------------------------------------------------------------
+def gen_config():
+    """Build the detector from the reference's examples/second config file, unchanged, through this repo's det3d (run before the
+    reference shims replace `det3d` in sys.modules)."""
+    from det3d.models import build_detector
+    from det3d.torchie import Config
+    cfg = Config.fromfile(os.path.join(REF, "examples", "second", "configs", "config.py"))
+    model = build_detector(cfg.model, train_cfg=cfg.train_cfg, test_cfg=cfg.test_cfg)
+    out = dict(model_type=cfg.model.type, out_size_factor=cfg.assigner.out_size_factor, test_cfg=json.loads(json.dumps(cfg.test_cfg)),
+               n_params=sum(p.numel() for p in model.parameters()))
+    sd = [[k, list(v.shape), str(v.dtype)] for k, v in model.state_dict().items()]
+    with open(os.path.join(HERE, "reference_config_detector.json"), "w") as f:       # one state-dict entry per line
+        f.write(json.dumps(out)[:-1] + ', "state_dict": [\n' + ",\n".join(json.dumps(e) for e in sd) + "\n]}\n")
+    print("config: %s, %d state-dict entries, %d parameters" % (out["model_type"], len(sd), out["n_params"]))
 
 
 # --------------------------------------------------------------------------------------------
@@ -372,6 +404,9 @@ if __name__ == "__main__":
         gen_voxel()
     if not only or "iou" in only:
         gen_iou()
+        gen_iou_self()
+    if "config" in only:             # imports this repo's det3d, which the shims below replace: run on its own (`make_golden.py config`)
+        gen_config()
     install_det3d_shims()
     if not only or "assign" in only:
         gen_anchors_assign()

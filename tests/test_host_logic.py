@@ -20,11 +20,16 @@ def test_library_loads_and_exports_every_declared_symbol():
     for name in declared:
         assert name in _lib.SIGNATURES, name             # the binding declares its signature
         assert hasattr(_lib.lib._prod, name), name       # and dlsym succeeds in the PRODUCT library
-    assert not _lib.lib.lab_loaded                       # importing / using the product does not load the lab library
     assert "sm_100a" in _lib.version()
     # no compute calls here (no GPU in this container): argument validation only
     assert _lib.lib.sessd_voxelize_workspace_bytes(20000, 1, None) == 0
     assert _lib.lib.sessd_nms_workspace_bytes(1000) == 8 * (1000 * 16 + 64)
+    # importing / using the product does not load the lab library: checked in a fresh interpreter, since GPU tests that run earlier in
+    # the same session load it on purpose
+    code = ("import sys; sys.path.insert(0, %r); from sessd_b200 import _lib; _lib.version(); "
+            "_lib.lib.sessd_voxelize_workspace_bytes(20000, 1, None); _lib.lib.sessd_nms_workspace_bytes(1000); "
+            "assert not _lib.lib.lab_loaded; assert 'libsessd_b200_lab' not in open('/proc/self/maps').read()") % os.path.join(ROOT, "se-ssd_b200")
+    subprocess.check_call([sys.executable, "-c", code])
 
 
 def test_lab_library_exports_every_declared_symbol_and_nothing_of_the_product():

@@ -31,18 +31,21 @@ def test_oracle_rotated_iou_equals_reference_golden_bit_exact(golden_dir):
     assert np.array_equal(ocpu.boxes_iou_bev(a5, c5), g["iou"])
 
 
-def test_oracle_matches_compiled_reference_when_present():
-    """oracle/_ref (reference iou3d_cpu.cpp compiled in place) travels with the repo; compare live if loadable."""
+def test_oracle_matches_compiled_reference_when_present(golden_dir):
+    """The reference's iou3d_cpu.cpp on 150 seeded boxes against themselves, bit-exact: always against its recorded output
+    (tests/golden/iou_self_case.npz), and live as well when oracle/_ref holds the reference compiled in place."""
     from oracle import build as obuild, cpu as ocpu
     from sessd_b200 import synth
+    b, _ = synth.random_boxes(99, 150, spread=0.2)
+    a5 = ocpu.boxes3d_to_bev(b)
+    got = ocpu.boxes_iou_bev(a5, a5)
+    assert np.array_equal(got, np.load(os.path.join(golden_dir, "iou_self_case.npz"))["iou"])
     ref = obuild.load_ref()
     if ref is None:
         return
-    b, _ = synth.random_boxes(99, 150, spread=0.2)
-    a5 = ocpu.boxes3d_to_bev(b)
     out = torch.zeros(150, 150)
     ref.boxes_iou_bev_cpu(torch.from_numpy(a5), torch.from_numpy(a5), out)
-    assert np.array_equal(out.numpy(), ocpu.boxes_iou_bev(a5, a5))
+    assert np.array_equal(out.numpy(), got)
 
 
 def test_oracle_anchors_and_assigner_equal_reference_golden(golden_dir):
